@@ -8,6 +8,8 @@ one pass of the hot path over that batch.
   python bench.py --gpus N --steps K --warmup W            (our CUDA path)
   python bench.py --impl reference ...                     (CPU reference arm:
         the oracle port of the reference's rasteriser on all host cores)
+  python bench.py ... --dump-outputs DIR                   (also writes the outputs of
+        the last timed step as .npy files, to compare two builds: dump_outputs)
 
 Prints ONE JSON line (rank 0).  See DESIGN.md "Measurement" for the definition
 of every field.
@@ -79,6 +81,21 @@ def pin_to_gpu_numa_node(local):
     except Exception as ex:                                  # not fatal: report and carry on unpinned
         return {"error": repr(ex)}
     return {"cpus": 0}
+
+
+DUMP_ALLMAP_SAMPLE = 1 << 22
+
+
+def dump_outputs(out_dir, color, allmap, radii, grad):
+    """Writes what the last timed step returned as <out_dir>/<name>.npy in float32 (43 MB in all): color [B,V,3,H,W],
+    radii [B,V,P] and the surfel gradient [B,P,13] whole, and allmap_sample, the allmap [B,V,7,H,W] values at a fixed
+    seeded sample of DUMP_ALLMAP_SAMPLE flat indices (sorted) -- the whole allmap alone would be 44 MB."""
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    idx = np.sort(np.random.default_rng(0).choice(allmap.numel(), DUMP_ALLMAP_SAMPLE, replace=False))
+    sample = allmap.reshape(-1)[torch.from_numpy(idx).to(allmap.device)]
+    for name, t in (("color", color), ("allmap_sample", sample), ("radii", radii), ("grad", grad)):
+        np.save(os.path.join(out_dir, name + ".npy"), t.detach().cpu().numpy().astype(np.float32))
 
 
 class ClockSampler:
@@ -281,6 +298,8 @@ def run_gpu(args):
     status = ws[L.status:L.status + 64].view(torch.int32).cpu()
     assert int(status[1]) == 0, "workspace overflow inside the timed region"
     assert torch.isfinite(grad).all()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, color, allmap, radii, grad)
     t = torch.tensor([dev_ms], device=dev, dtype=torch.float64)
     if world > 1:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -832,7 +851,13 @@ def main():
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--no-dit", action="store_true", help="skip the secondary DiT sampling legs (DiT, cascade, stand-ins)")
     ap.add_argument("--no-c5", action="store_true", help="skip the C5 decode -> all-gather -> render leg")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write rank 0's outputs of the last timed raster step to DIR/<name>.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the GPU path (--impl ours)")
     if args.impl == "reference":
         run_reference(args)
     else:

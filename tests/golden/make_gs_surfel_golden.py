@@ -15,9 +15,17 @@ it imports but this image lacks is stubbed:
     tensors on the CPU while the module is constructed.
 Only runs inside the build container (needs /root/reference); the .npz it writes is committed and is what
 tests/test_raster_gpu.py::test_reference_loop_golden compares the CUDA mirror with.
+
+It also writes gs_surfel_loop_calls.json: every call the reference's loop made to the rasteriser, in order -- which
+batch item and view it passed (checked here to be exactly the golden's `g` / `view` / `proj` at those indices), the
+background, scale modifier and image size, and sha256 digests of the raw (color, radii, allmap) the shim returned.
+The golden is the reference's post-processing of exactly those returns, so tests/test_round2_cpu.py pins the golden
+without the reference tree by replaying every call through the C oracle and comparing the digests.
     python tests/golden/make_gs_surfel_golden.py [--check]
 """
+import hashlib
 import importlib.util
+import json
 import os
 import sys
 import types
@@ -25,9 +33,8 @@ from typing import NamedTuple
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(os.path.dirname(HERE))
-sys.path.insert(0, HERE)
-sys.path.insert(0, ROOT)
-from _ref_stubs import *  # noqa: F401,F403,E402  (puts /root/reference on sys.path, installs the dummies)
+if ROOT not in sys.path:
+    sys.path.insert(0, ROOT)
 import numpy as np  # noqa: E402
 import torch  # noqa: E402
 
@@ -35,6 +42,8 @@ from oracle import surfel_oracle as so  # noqa: E402
 from tools import synth  # noqa: E402
 
 OUT = os.path.join(HERE, "gs_surfel_loop.npz")
+CALLS = os.path.join(HERE, "gs_surfel_loop_calls.json")
+_calls = []                                            # what the reference's loop passed to / got from the shim
 
 
 # ---- oracle-backed stand-in for the un-vendored third-party module --------------------------------------------
@@ -65,10 +74,17 @@ class GaussianRasterizer(torch.nn.Module):
         o = so.rasterize(means3D.numpy(), opacities.numpy(), scales.numpy(), rotations.numpy(), colors_precomp.numpy(),
                          rs.viewmatrix.numpy(), rs.projmatrix.numpy(), rs.bg.numpy(), int(rs.image_height),
                          int(rs.image_width), float(rs.scale_modifier))
+        assert rs.image_height == rs.image_width
+        _calls.append(dict(g13=torch.cat([means3D, opacities, scales, rotations, colors_precomp], 1).numpy(),
+                           view=rs.viewmatrix.numpy().copy(), proj=rs.projmatrix.numpy().copy(), bg=rs.bg.numpy().copy(),
+                           scale_modifier=float(rs.scale_modifier), size=int(rs.image_height),
+                           color=o["color"], radii=o["radii"], allmap=o["allmap"]))
         return torch.from_numpy(o["color"]), torch.from_numpy(o["radii"]), torch.from_numpy(o["allmap"])
 
 
 def load_reference_renderer():
+    sys.path.insert(0, HERE)
+    import _ref_stubs  # noqa: F401  (puts the reference tree on sys.path, installs the dummies)
     shim = types.ModuleType("diff_surfel_rasterization")
     shim.GaussianRasterizationSettings = GaussianRasterizationSettings
     shim.GaussianRasterizer = GaussianRasterizer
@@ -115,16 +131,41 @@ def generate():
         for k, v in r.items():
             out["%s__%s" % (tag, k)] = v.numpy().astype(np.float32)
     out["b__bg"] = bg.numpy()
-    return out
+    return out, recorded_calls(g, cam["view"], cam["proj"])
+
+
+def digest(a):
+    """sha256 of an array's dtype, shape and bytes: a bit-exact pin that stays small."""
+    a = np.ascontiguousarray(a)
+    return hashlib.sha256(("%s %s " % (a.dtype.str, a.shape)).encode() + a.tobytes()).hexdigest()
+
+
+def recorded_calls(g, view, proj):
+    """The shim's record; each call is tied to the one (batch item, view) of the golden inputs it was given."""
+    rec = []
+    for i, c in enumerate(_calls):
+        hits = [(b, v) for b in range(view.shape[0]) for v in range(view.shape[1])
+                if np.array_equal(c["g13"], g[b]) and np.array_equal(c["view"], view[b, v])
+                and np.array_equal(c["proj"], proj[b, v])]
+        assert len(hits) == 1, (i, hits)
+        rec.append({"item": hits[0][0], "view": hits[0][1], "bg": [float(x) for x in c["bg"]],
+                    "scale_modifier": c["scale_modifier"], "size": c["size"],
+                    "sha256": {k: digest(c[k]) for k in ("color", "radii", "allmap")}})
+    return rec
 
 
 if __name__ == "__main__":
-    new = generate()
+    new, calls = generate()
     if "--check" in sys.argv:
         old = np.load(OUT)
         for k in new:
             assert np.array_equal(np.asarray(new[k]), old[k]), k
-        print("golden reproduces bit for bit:", OUT)
+        with open(CALLS) as f:
+            assert json.load(f) == calls, CALLS
+        print("golden reproduces bit for bit:", OUT, CALLS)
     else:
         np.savez_compressed(OUT, **new)
-        print("wrote", OUT, os.path.getsize(OUT), "bytes")
+        with open(CALLS, "w") as f:
+            json.dump(calls, f, indent=1)
+            f.write("\n")
+        print("wrote", OUT, os.path.getsize(OUT), "bytes and", CALLS)

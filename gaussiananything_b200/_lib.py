@@ -50,6 +50,9 @@ def lib():
     L.ga_raster_forward_async.restype = i32
     L.ga_raster_backward_scratch_bytes.argtypes = [i32, i32, i32]
     L.ga_raster_backward_scratch_bytes.restype = sz
+    L.ga_raster_backward_records.argtypes = [i32, i32, i32, i32, i32, vp, sz, i64, i32, vp, sz,
+                                             C.POINTER(C.c_uint64), C.POINTER(C.c_uint64), vp]
+    L.ga_raster_backward_records.restype = i32
     L.ga_raster_backward.argtypes = [vp, i32, i32, i32, vp, vp, vp, i32, i32, f32,
                                      vp, vp, vp, vp, sz, i64, vp, sz, vp, vp]
     L.ga_raster_backward.restype = i32

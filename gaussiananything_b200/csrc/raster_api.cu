@@ -247,6 +247,17 @@ extern "C" int ga_raster_forward_render(const float *gauss13, int batch, int P, 
 #endif
 static size_t bwd_acc_bytes(int batch, int P, int views) { return align_up((size_t)batch * views * P * GA_GRAD_F * sizeof(float), 256); }
 static size_t bwd_tiles_bytes(int batch, int views) { return align_up(((size_t)batch * views * 255 * 255 + 1) * sizeof(uint32_t), 256); }
+// scratch bytes in front of the record lists: accumulators | tile slice starts | flag
+static size_t bwd_fixed_bytes(int batch, int P, int views) { return bwd_acc_bytes(batch, P, views) + bwd_tiles_bytes(batch, views) + 256; }
+// records the split backward's lists hold in `scratch_bytes`; 0: the buffer holds (little more than) the accumulators and
+// the fused kernel is chosen on the host
+static uint32_t bwd_list_capacity(int batch, int P, int views, size_t scratch_bytes)
+{
+    const size_t fixed = bwd_fixed_bytes(batch, P, views);
+    if (scratch_bytes <= fixed + 4096) return 0;
+    const size_t cap = (scratch_bytes - fixed) / 16;
+    return (uint32_t)(cap > 0xfffffff0ull ? 0xfffffff0ull : cap);
+}
 
 extern "C" size_t ga_raster_backward_scratch_bytes(int batch, int P, int views)
 {
@@ -299,13 +310,12 @@ extern "C" int ga_raster_backward_ex(const float *gauss13, int batch, int P, int
     BwdLists lists = {};
     {
         // a caller that passes only the accumulators (the round-1 scratch size) gets the fused kernel
-        const size_t fixed = need + bwd_tiles_bytes(batch, views) + 256;
-        if (scratch_bytes > fixed + 4096) {
+        const uint32_t cap = bwd_list_capacity(batch, P, views, scratch_bytes);
+        if (cap > 0) {
             char *p = (char *)scratch + need;
             lists.tile_rec_start = (uint32_t *)p;
             lists.records = (uint4 *)(p + bwd_tiles_bytes(batch, views) + 256);
-            const size_t cap = (scratch_bytes - fixed) / 16;
-            lists.capacity = (uint32_t)(cap > 0xfffffff0ull ? 0xfffffff0ull : cap);
+            lists.capacity = cap;
             lists.inst_off = w.inst_off;
             lists.inst_cnt = w.inst_cnt;
             const size_t mi = (size_t)(max_instances > 0 ? max_instances : 1);
@@ -317,6 +327,43 @@ extern "C" int ga_raster_backward_ex(const float *gauss13, int batch, int P, int
     if ((e = ga_launch_preprocess_bwd(d, w, gauss13, viewmats, projmats, radii, grad_acc, grad_gauss13, s)) != cudaSuccess)
         return (int)e;
     prof(6, s);
+    return 0;
+}
+
+extern "C" int ga_raster_backward_records(int batch, int P, int views, int H, int W,
+                                          const void *workspace, size_t workspace_bytes, int64_t max_instances,
+                                          int list_k, void *scratch, size_t scratch_bytes,
+                                          uint64_t *total, uint64_t *capacity, void *stream)
+{
+    RasterDims d;
+    int rc = make_dims(batch, P, views, H, W, 1.0f, max_instances, &d, list_k);
+    if (rc) return rc;
+    if (!workspace || !total || !capacity) return GA_ERR_BADARG;
+    GaRasterLayout L;
+    ga_raster_layout_ex(batch, P, views, H, W, max_instances, list_k, &L);
+    if (workspace_bytes < L.total_bytes) return GA_ERR_WORKSPACE;
+    RasterWs w;
+    carve(L, const_cast<void *>(workspace), &w);
+    cudaStream_t s = (cudaStream_t)stream;
+    cudaError_t e;
+    const uint32_t *dev_total;
+    if (list_k > 0) {
+        dev_total = w.tile_rec_start + (size_t)d.NV * d.T;                  // laid out by the forward
+    } else {
+        // the slice layout the backward would compute, in the same place of the scratch
+        if (!scratch || scratch_bytes < bwd_fixed_bytes(batch, P, views)) return GA_ERR_WORKSPACE;
+        uint32_t *trs = (uint32_t *)((char *)scratch + bwd_acc_bytes(batch, P, views));
+        if ((e = ga_launch_bwd_slices(d, w, trs, s)) != cudaSuccess) return (int)e;
+        dev_total = trs + (size_t)d.NV * d.T;
+    }
+    int32_t overflow = 0;
+    uint32_t t32 = 0;
+    if ((e = cudaMemcpyAsync(&overflow, w.status + 1, sizeof(int32_t), cudaMemcpyDeviceToHost, s)) != cudaSuccess) return (int)e;
+    if ((e = cudaMemcpyAsync(&t32, dev_total, sizeof(uint32_t), cudaMemcpyDeviceToHost, s)) != cudaSuccess) return (int)e;
+    if ((e = cudaStreamSynchronize(s)) != cudaSuccess) return (int)e;
+    if (overflow) return GA_ERR_WORKSPACE;                                    // the forward binned nothing
+    *total = t32;
+    *capacity = bwd_list_capacity(batch, P, views, scratch_bytes);
     return 0;
 }
 

@@ -103,6 +103,8 @@ cudaError_t ga_launch_render_fwd_with_slices(const RasterDims &d, const RasterWs
 cudaError_t ga_launch_render_bwd(const RasterDims &d, const RasterWs &w, const float *bg,
                                  const float *dL_dcolor, const float *dL_dallmap,
                                  float *grad_acc, const BwdLists &lists, cudaStream_t s);
+// per-tile record totals of the split backward and their scan into tile_rec_start[NV*T + 1] ([NV*T] = total)
+cudaError_t ga_launch_bwd_slices(const RasterDims &d, const RasterWs &w, uint32_t *tile_rec_start, cudaStream_t s);
 cudaError_t ga_launch_preprocess_bwd(const RasterDims &d, const RasterWs &w, const float *gauss13,
                                      const float *viewmats, const float *projmats,
                                      const int32_t *radii, const float *grad_acc,

@@ -75,6 +75,19 @@ __device__ __forceinline__ bool eval_pair(const float4 a, const float4 b, const 
     return o.alpha >= 1.0f / 255.0f;
 }
 
+// pixels of the tile with origin (ox, oy) inside the cull box bb = (x0, x1, y0, y1): the record-slice length of an
+// instance in the split backward, and an upper bound of its list length in the fused one.  An empty box (a surfel
+// too transparent to reach alpha 1/255 anywhere: +-1e30 bounds) has no pixel.  The bounds are clamped to one pixel
+// beyond the tile, which changes no count: unclamped, +-1e30 saturates the float -> int conversions and the wrapped
+// difference counts 2 x 2 pixels.
+__device__ __forceinline__ int clipped_box_area(const float4 bb, int ox, int oy)
+{
+    const float x0 = fminf(fmaxf(bb.x, (float)ox), (float)(ox + 16)), x1 = fmaxf(fminf(bb.y, (float)(ox + 15)), (float)(ox - 1));
+    const float y0 = fminf(fmaxf(bb.z, (float)oy), (float)(oy + 16)), y1 = fmaxf(fminf(bb.w, (float)(oy + 15)), (float)(oy - 1));
+    const int wx = max(0, (int)floorf(x1) - (int)ceilf(x0) + 1), wy = max(0, (int)floorf(y1) - (int)ceilf(y0) + 1);
+    return wx * wy;
+}
+
 // Forward staging record (tile-local, computed once per (tile, surfel) by the
 // staging thread): with o = tile origin, k_o = o.x*Tw - Tu, l_o = o.y*Tw - Tv,
 //   p(dx,dy) = (k_o + dx*Tw) x (l_o + dy*Tw) = C + dx*A + dy*B,
@@ -106,13 +119,14 @@ render_fwd_kernel(RasterDims d, RasterWs ws, const float *__restrict__ bg,
     constexpr int GW = GS == 32 ? 8 : 4;                         // group block width / height in pixels
     constexpr int GH = GS == 8 ? 2 : 4;
     __shared__ float4 s_rec[7][CHUNK];
-    __shared__ uint32_t s_area;                                  // LISTS: sum of the clipped cull-box areas staged so far
+    __shared__ uint32_t s_area;                                  // LISTS: sum of the clipped cull-box areas of this chunk
+    __shared__ unsigned long long s_area_sum;                    // ... and of all chunks staged so far (thread 0)
     if (ws.status[1]) return;
     const int view = blockIdx.z;
     const int tile = blockIdx.y * d.gx + blockIdx.x;
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const int grp = lane / GS, gl = lane % GS;
-    if (LISTS && threadIdx.x == 0) s_area = 0;
+    if (LISTS && threadIdx.x == 0) { s_area = 0; s_area_sum = 0; }
     const int ox = blockIdx.x * GA_BLOCK_X, oy = blockIdx.y * GA_BLOCK_Y;
     const int wx0 = (warp & 1) * 8, wy0 = (warp >> 1) * 4;       // warp's 8x4 block, tile-local
     // group blocks tile the warp block: GS=16 -> 2 side by side (4x4); GS=8 -> 2x2 arrangement of 4x2 blocks
@@ -158,14 +172,7 @@ render_fwd_kernel(RasterDims d, RasterWs ws, const float *__restrict__ bg,
             s_rec[4][threadIdx.x] = make_float4(bb.x - oxf, bb.y - oxf, bb.z - oyf, bb.w - oyf);
             s_rec[5][threadIdx.x] = nr;
             s_rec[6][threadIdx.x] = gb;
-            if (LISTS) {
-                // slice length of this instance in the backward's record buffer = pixels of its cull box inside the tile
-                // (same formula as clipped_box_area(): box and tile in absolute coordinates)
-                const float x0 = fmaxf(bb.x, oxf), x1 = fminf(bb.y, oxf + 15.f);
-                const float y0 = fmaxf(bb.z, oyf), y1 = fminf(bb.w, oyf + 15.f);
-                const int wx = max(0, (int)floorf(x1) - (int)ceilf(x0) + 1), wy = max(0, (int)floorf(y1) - (int)ceilf(y0) + 1);
-                area = (uint32_t)(wx * wy);
-            }
+            if (LISTS) area = (uint32_t)clipped_box_area(bb, ox, oy);    // slice length in the backward's record buffer
         }
         if (LISTS) {
 #pragma unroll
@@ -173,6 +180,9 @@ render_fwd_kernel(RasterDims d, RasterWs ws, const float *__restrict__ bg,
             if (lane == 0 && area) atomicAdd(&s_area, area);
         }
         __syncthreads();
+        // 64-bit running sum (a tile of 2^24 full-tile instances reaches 2^32); s_area is next written after the
+        // barrier at the top of the loop
+        if (LISTS && threadIdx.x == 0) { s_area_sum += s_area; s_area = 0; }
         for (int g0 = 0; g0 < cnt; g0 += 32) {
             if (__all_sync(0xffffffffu, done)) break;
             const int j = g0 + lane;
@@ -251,7 +261,7 @@ render_fwd_kernel(RasterDims d, RasterWs ws, const float *__restrict__ bg,
         if (nl > d.list_k) ws.tile_flag[(size_t)view * d.T + tile] = 1u;      // this tile's backward recomputes
         // every chunk the backward can reach (positions below the last contributor) has been staged here, so the sum
         // covers its slices; bwd_scan_area_kernel turns the per-tile sums into offsets
-        if (threadIdx.x == 0) ws.tile_rec_start[(size_t)view * d.T + tile] = s_area;
+        if (threadIdx.x == 0) ws.tile_rec_start[(size_t)view * d.T + tile] = (uint32_t)min(s_area_sum, 0xffffffffull);
     }
     if (inside) {
         const size_t HW = (size_t)d.H * d.W;
@@ -563,10 +573,7 @@ render_bwd_kernel(RasterDims d, RasterWs ws, const float *__restrict__ bg,
 #pragma unroll
             for (int k = 0; k < 6; k++) { q[k] = __ldg(src + k); sm.rec[k][threadIdx.x] = q[k]; }
             // pixels of this tile inside the cull box (upper bound of the surfel's list length)
-            const float x0 = fmaxf(q[4].x, (float)ox), x1 = fminf(q[4].y, (float)(ox + 15));
-            const float y0 = fmaxf(q[4].z, (float)oy), y1 = fminf(q[4].w, (float)(oy + 15));
-            const int wx = max(0, (int)floorf(x1) - (int)ceilf(x0) + 1), wy = max(0, (int)floorf(y1) - (int)ceilf(y0) + 1);
-            const int area = wx * wy;
+            const int area = clipped_box_area(q[4], ox, oy);
             big0 = area > BWD_LIST_RECORDS / 128; big1 = area > BWD_LIST_RECORDS / 64;
             big2 = area > BWD_LIST_RECORDS / 32; big3 = area > BWD_LIST_RECORDS / 16;
         }
@@ -674,14 +681,6 @@ render_bwd_kernel(RasterDims d, RasterWs ws, const float *__restrict__ bg,
 // tile totals.  If the total exceeds the buffer, a device flag routes the launch to the fused kernel instead (no
 // host synchronisation either way).  Extra traffic: 16 B written + read per record, ~2 x 26 M records on C2.
 // ---------------------------------------------------------------------------
-__device__ __forceinline__ int clipped_box_area(const float4 bb, int ox, int oy)
-{
-    const float x0 = fmaxf(bb.x, (float)ox), x1 = fminf(bb.y, (float)(ox + 15));
-    const float y0 = fmaxf(bb.z, (float)oy), y1 = fminf(bb.w, (float)(oy + 15));
-    const int wx = max(0, (int)floorf(x1) - (int)ceilf(x0) + 1), wy = max(0, (int)floorf(y1) - (int)ceilf(y0) + 1);
-    return wx * wy;
-}
-
 // one warp per tile: sum of the clipped cull-box areas of the tile's instances
 __global__ void __launch_bounds__(256)
 bwd_tile_area_kernel(RasterDims d, RasterWs ws, uint32_t *__restrict__ tile_rec_start)
@@ -694,22 +693,26 @@ bwd_tile_area_kernel(RasterDims d, RasterWs ws, uint32_t *__restrict__ tile_rec_
     const int ox = (tile % d.gx) * GA_BLOCK_X, oy = (tile / d.gx) * GA_BLOCK_Y;
     const uint32_t start = ws.tile_start[t], end = ws.tile_start[t + 1];
     const float *rec_base = ws.rec + (size_t)view * d.P * GA_REC_F;
-    uint32_t sum = 0;
+    // 64-bit: up to 256 records per instance, so 2^24 instances of one tile reach 2^32
+    unsigned long long sum = 0;
     for (uint32_t i = start + lane; i < end; i += 32) {
         const float4 bb = __ldg(reinterpret_cast<const float4 *>(rec_base + (size_t)ws.ids[i] * GA_REC_F) + 4);
-        sum += (uint32_t)clipped_box_area(bb, ox, oy);
+        sum += (unsigned long long)clipped_box_area(bb, ox, oy);
     }
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) sum += __shfl_xor_sync(0xffffffffu, sum, o);
-    if (lane == 0) tile_rec_start[t] = sum;
+    if (lane == 0) tile_rec_start[t] = (uint32_t)min(sum, 0xffffffffull);     // saturated: the total saturates too
 }
 
-// exclusive scan of the tile totals (one block); sets the fallback flag when the buffer is too small
+// exclusive scan of the tile totals (one block); sets the fallback flag when the buffer is too small.  The scan runs
+// in 64 bits and the total is stored saturated at 0xffffffff, above every capacity (<= 0xfffffff0): a total that
+// wrapped at 2^32 could look small enough for the buffer.  The offsets themselves stay 32-bit -- they are only used
+// when the total fits the buffer.
 __global__ void __launch_bounds__(1024)
 bwd_scan_area_kernel(RasterDims d, RasterWs ws, uint32_t *__restrict__ tile_rec_start)
 {
-    __shared__ uint32_t s_warp[32];
-    __shared__ uint32_t s_carry;
+    __shared__ unsigned long long s_warp[32];
+    __shared__ unsigned long long s_carry;
     if (ws.status[1]) return;
     const int n = d.NV * d.T;
     if (threadIdx.x == 0) s_carry = 0;
@@ -717,33 +720,34 @@ bwd_scan_area_kernel(RasterDims d, RasterWs ws, uint32_t *__restrict__ tile_rec_
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     for (int base = 0; base < n; base += 1024) {
         const int i = base + threadIdx.x;
-        const uint32_t v = i < n ? tile_rec_start[i] : 0u;
-        uint32_t x = v;
+        const unsigned long long v = i < n ? tile_rec_start[i] : 0u;
+        unsigned long long x = v;
 #pragma unroll
         for (int o = 1; o < 32; o <<= 1) {
-            const uint32_t y = __shfl_up_sync(0xffffffffu, x, o);
+            const unsigned long long y = __shfl_up_sync(0xffffffffu, x, o);
             if (lane >= o) x += y;
         }
         if (lane == 31) s_warp[warp] = x;
         __syncthreads();
         if (warp == 0) {
-            const uint32_t wv = s_warp[lane];
-            uint32_t wx = wv;
+            const unsigned long long wv = s_warp[lane];
+            unsigned long long wx = wv;
 #pragma unroll
             for (int o = 1; o < 32; o <<= 1) {
-                const uint32_t y = __shfl_up_sync(0xffffffffu, wx, o);
+                const unsigned long long y = __shfl_up_sync(0xffffffffu, wx, o);
                 if (lane >= o) wx += y;
             }
             s_warp[lane] = wx - wv;
         }
         __syncthreads();
-        const uint32_t excl = s_carry + s_warp[warp] + x - v;
-        if (i < n) tile_rec_start[i] = excl;
+        const unsigned long long excl = s_carry + s_warp[warp] + x - v;
+        if (i < n) tile_rec_start[i] = (uint32_t)excl;
         __syncthreads();
         if (threadIdx.x == 1023) s_carry = excl + v;
         __syncthreads();
     }
-    if (threadIdx.x == 0) tile_rec_start[n] = s_carry;     // total records needed; > capacity -> the fused kernel runs instead
+    // total records needed; > capacity -> the fused kernel runs instead
+    if (threadIdx.x == 0) tile_rec_start[n] = (uint32_t)min(s_carry, 0xffffffffull);
 }
 
 // the record buffer of the split backward is too small for this launch: every split kernel exits, the fused one runs

@@ -3,7 +3,8 @@
  * paths of GaussianAnything.  Plain pointers and sizes only; no torch types.
  *
  * All pointers are DEVICE pointers unless stated otherwise.  No entry point
- * allocates, frees or synchronises; everything is enqueued on `stream`
+ * allocates, frees or synchronises (except the ga_raster_backward_records
+ * probe, which returns a device count); everything is enqueued on `stream`
  * (a cudaStream_t passed as void*).  Return value: 0 on success, a negative
  * GA_ERR_* code on a bad argument, or a positive cudaError_t from the launch.
  *
@@ -167,6 +168,21 @@ int ga_raster_set_tuning(int fwd_group);
  * the split backward (64 records of 16 bytes per (surfel, view)).  A smaller buffer that still holds the
  * accumulators is accepted: the backward then runs its fused shared-memory kernel. */
 size_t ga_raster_backward_scratch_bytes(int batch, int P, int views);
+
+/*
+ * Which backward a scratch buffer gets, and the record budget a scene needs.  *total = the number of 16-byte records
+ * the split backward would lay out for the forward in `workspace` -- the value it compares with its capacity on the
+ * device -- and *capacity = the records `scratch_bytes` of scratch provide (0: the buffer holds no more than the
+ * accumulators, tile table and 4 KB, and the fused kernel is chosen on the host).  total <= capacity: the split
+ * kernels run; total > capacity: the fused kernel runs instead.  list_k > 0 reads the layout the forward computed;
+ * list_k == 0 computes it into `scratch` exactly as ga_raster_backward_ex would (the scratch must then hold at least
+ * the accumulators and the tile table).  Unlike every other entry point this one synchronises `stream` and copies
+ * the total to the host.  GA_ERR_WORKSPACE when the forward overflowed its workspace.
+ */
+int ga_raster_backward_records(int batch, int P, int views, int H, int W,
+                               const void *workspace, size_t workspace_bytes, int64_t max_instances, int list_k,
+                               void *scratch, size_t scratch_bytes, uint64_t *total, uint64_t *capacity,
+                               void *stream);
 
 /*
  * Backward.  dL_dcolor [NV][3][H][W], dL_dallmap [NV][7][H][W]; grad_gauss13
